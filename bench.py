@@ -27,6 +27,13 @@ memory inside the timed region.  Riding along in the same line:
 "cpu_baseline" and `--impl reference` time the CPU restatement of the reference path (oracle/) on a
 bounded sample: median of 3 repeats, thread sweep including the reference's default of 8 threads.
 Only the JSON line goes to stdout.
+
+`--dump-outputs DIR` writes, after the timed loops, what each timed path computed in its last timed step as
+DIR/<name>.npy (float32 / float64, integers stored exactly): the factor tables after the last timed ALS epoch
+(a fixed, seeded sample of rows), the item-kNN similarity matrix of the last timed build (CSR), and a seeded
+sample of query rows of the last scoring launch (scores with 0 where an item is unscored, a 0/1 mask of the
+scored items, and neighbour counts).  Inputs are seeded, so two builds of the project run with the
+same arguments can be compared output for output.
 """
 
 from __future__ import annotations
@@ -361,6 +368,29 @@ def run_reference(args, rank: int) -> None:
 _JSON_OUT = None
 
 
+DUMP_LIMIT = 64 << 20  # bytes written by --dump-outputs in all
+DUMP_ROWS = 16384  # sampled rows per factor table
+
+
+def sample_rows(n: int, k: int, seed: int) -> np.ndarray:
+    """A fixed, sorted sample of ``min(n, k)`` row indices."""
+    return np.sort(np.random.default_rng(seed).choice(n, min(n, k), replace=False))
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """``--dump-outputs``: one ``<name>.npy`` per array, finite float32 / float64 only, within DUMP_LIMIT."""
+    total = sum(np.asarray(a).nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        assert np.isfinite(a).all(), f"--dump-outputs: {name} is not finite"
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+    log(f"[bench] wrote {len(arrays)} arrays ({total} bytes) to {out_dir}")
+
+
 def emit(line: dict) -> None:
     """The one JSON line goes to the real stdout; everything else (NCCL's version banner, library
     chatter written to fd 1) was redirected to stderr by main()."""
@@ -493,6 +523,8 @@ def main() -> None:
     ap.add_argument("--variants", default="bf16,fp32", help="ALS gather dtypes to time (profiling runs pass one)")
     ap.add_argument("--profile", action="store_true", help="under ncu: honour a small --warmup, skip e2e/parity/CPU")
     ap.add_argument("--scale", type=float, default=1.0, help="scale-out workloads: fraction of the full size (smoke runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed paths computed in their last timed step to DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 0)
     if args.profile:
@@ -548,6 +580,7 @@ def main() -> None:
 
     results: dict = {}
     parity: dict = {}
+    dumped: dict = {}  # --dump-outputs, rank 0
     launches = 0
     variants = [v for v in args.variants.split(",") if v]
     for tag, gdt in (("bf16", "bfloat16"), ("fp32", "float32")):
@@ -582,6 +615,11 @@ def main() -> None:
         barrier()
         t_end = time.time()
         clocks = sampler.stop(t_begin, t_end) if (rank == 0 and tag == "bf16") else None
+        if args.dump_outputs and rank == 0:  # the factors as the last timed epoch left them
+            for side, t, seed in (("user", tr.d_users, 1), ("item", tr.d_items, 2)):
+                rows = torch.from_numpy(sample_rows(t.shape[0], DUMP_ROWS, seed)).to(t.device)
+                dumped[f"als_{tag}_{side}_rows"] = rows.cpu().numpy().astype(np.float64)
+                dumped[f"als_{tag}_{side}_factors"] = t.index_select(0, rows).float().cpu().numpy()
         # the same epochs once more with CUDA events around every row-solve launch (the roofline's
         # kernel time; events cannot sit inside a captured graph, so this loop launches eagerly)
         tr.kernel_events = []
@@ -696,7 +734,7 @@ def main() -> None:
 
     knn = None
     if not args.no_knn:
-        knn = bench_knn(args, inter, dev, peak, peak_src, rank, world, parity)
+        knn = bench_knn(args, inter, dev, peak, peak_src, rank, world, parity, dumped if args.dump_outputs else None)
 
     cpu = None
     if not args.no_cpu and rank == 0 and world == 1:
@@ -722,6 +760,8 @@ def main() -> None:
         for k_ in ("_kui", "_kiu", "_cost"):
             knn.pop(k_, None)
 
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dumped)
     ok = all(v.get("ok", True) for v in parity.values()) if parity else None
     if rank == 0:
         head = results.get("bf16") or results["fp32"]
@@ -757,6 +797,12 @@ def main() -> None:
         raise SystemExit(1)
 
 
+def dump_csr(dumped: dict, name: str, indptr, cols, vals) -> None:
+    dumped[f"{name}_indptr"] = indptr.cpu().numpy().astype(np.float64)
+    dumped[f"{name}_cols"] = cols.cpu().numpy().astype(np.float64)
+    dumped[f"{name}_vals"] = vals.cpu().numpy().astype(np.float32)
+
+
 def bench_recommend(args, tr, dev, peak, peak_src) -> dict:
     """
     SURVEY.md §8f N1/N2: top-100 of all items for a batch of users from the factors just trained —
@@ -776,7 +822,7 @@ def bench_recommend(args, tr, dev, peak, peak_src) -> dict:
     engine.topn_columns(s, n_top)
     torch.cuda.synchronize()
     ev = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
-    reps = 3
+    reps = args.steps
     t_gemm = t_top = 0.0
     for _ in range(reps):
         ev[0].record()
@@ -824,7 +870,7 @@ def bench_recommend(args, tr, dev, peak, peak_src) -> dict:
     return out
 
 
-def bench_knn(args, inter, dev, peak, peak_src, rank: int, world: int, parity: dict) -> dict | None:
+def bench_knn(args, inter, dev, peak, peak_src, rank: int, world: int, parity: dict, dumped: dict | None = None) -> dict | None:
     import torch
 
     from lkpy_b200 import accel, data, engine
@@ -861,6 +907,16 @@ def bench_knn(args, inter, dev, peak, peak_src, rank: int, world: int, parity: d
             sc, ct = st.score_all_items(ref_ptr, d_ri[a0:a1], d_rv[a0:a1], KNN_MAX_NBRS, 1)
             e1.record()
             torch.cuda.synchronize()
+            if dumped is not None and rank == 0 and u1 == u_end:  # the last launch: a fixed sample of its queries
+                rows = sample_rows(u1 - u0, 32, 3)
+                dumped["knn_score_users"] = (u0 + rows).astype(np.float64)
+                d_rows = torch.from_numpy(rows).to(dev)
+                # an item without enough neighbours has no score (NaN): 0 there, and the mask says which are scored
+                scores = sc.index_select(0, d_rows).cpu().numpy()
+                has_score = ~np.isnan(scores)
+                dumped["knn_score_scores"] = np.where(has_score, scores, np.float32(0.0))
+                dumped["knn_score_scored"] = has_score.astype(np.float32)
+                dumped["knn_score_counts"] = ct.index_select(0, d_rows).cpu().numpy().astype(np.float32)
             total_ms += e0.elapsed_time(e1)
             scored += u1 - u0
             touched += int(row_len[R.indices[a_lo + a0 : a_lo + a1]].sum())
@@ -897,7 +953,7 @@ def bench_knn(args, inter, dev, peak, peak_src, rank: int, world: int, parity: d
         sbuild()
         dist.barrier()
         torch.cuda.synchronize()
-        reps = max(1, min(args.steps, 3))
+        reps = args.steps
         s0, s1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         s0.record()
         for _ in range(reps):
@@ -909,6 +965,8 @@ def bench_knn(args, inter, dev, peak, peak_src, rank: int, world: int, parity: d
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
         extra = None
+        if dumped is not None and rank == 0:
+            dump_csr(dumped, "knn_sim", *engine.topk_rows_to_csr(cols, vals, cnt))
         if not args.no_parity:
             from oracle import parity as par
 
@@ -971,7 +1029,7 @@ def bench_knn(args, inter, dev, peak, peak_src, rank: int, world: int, parity: d
 
     plan, csr = build()  # warm-up (also loads the kernels)
     torch.cuda.synchronize()
-    reps = max(1, min(args.steps, 3))
+    reps = args.steps
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     k0, k1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
@@ -980,6 +1038,8 @@ def bench_knn(args, inter, dev, peak, peak_src, rank: int, world: int, parity: d
     e1.record()
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / reps
+    if dumped is not None:
+        dump_csr(dumped, "knn_sim", *csr)
     # the accumulate kernel alone (same stream, events around the launch)
     import ctypes as C
 
